@@ -2,7 +2,7 @@
 """bench.py - forward+backward throughput of the rasterizer hot path (BASELINE.json metric:
 "fwd+bwd Mpix/s @1M Gaussians/1024^2; HBM GB/s vs roofline; 1/2/4/8 GPU").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one view of the workload rendered (forward) and back-propagated (backward) through
 the public drop-in API (GaussianRasterizer -> C ABI -> sm_100a kernels).  N>1 (torchrun, one
@@ -14,6 +14,8 @@ Prints ONE JSON line (rank 0).  See the task contract for the keys; additions:
   cpu_baseline  the pure-PyTorch CPU oracle timed on this box on a bounded sample (N=1 only)
   stages_ms     mean device time of every kernel stage over the timed steps
 --impl reference times the CPU oracle port (the reference's CUDA op is un-vendored; DESIGN.md).
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (rank 0;
+see dump_sample), so that two builds can be compared output for output on identical inputs.
 """
 from __future__ import annotations
 
@@ -228,6 +230,24 @@ def run_reference(args, wl_name, wl, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_ROWS = 1 << 16                  # per-Gaussian outputs are sampled: 1M full rows would be ~250 MB
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_sample(color, radii, da, grads, P):
+    """Host copy of one step's results as its caller receives them: the rendered colour [3,H,W] and
+    depth/alpha [2,H,W] in full; radii and the gradients of every input on DUMP_ROWS Gaussians drawn
+    with a fixed seed (their indices are written as sample_index).  All float32 or float64."""
+    idx = np.sort(np.random.RandomState(0).choice(P, min(P, DUMP_ROWS), replace=False))
+    sel = torch.from_numpy(idx).to(color.device)
+    out = {"color": color, "depth_alpha": da, "radii": radii.index_select(0, sel).float()}
+    out.update({f"grad_{k}": g.index_select(0, sel) for k, g in grads.items()})
+    out = {k: v.detach().cpu().numpy() for k, v in out.items()}
+    out["sample_index"] = idx.astype(np.float64)
+    assert sum(v.nbytes for v in out.values()) <= DUMP_MAX_BYTES
+    return out
+
+
 def workload_config(wl_name, wl, world, sh_degree=3):
     """The `config` object both arms print (identical keys, so the driver sees the same config)."""
     return {"workload": wl_name, "P": wl["P"], "H": wl["H"], "W": wl["W"], "sh_degree": sh_degree, "M": 16,
@@ -286,7 +306,11 @@ def main():
                          "(all-gather, rebuilt locally) or all-reduced as [P,M,3] rows")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     wl_name, wl = args.workload, WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -345,7 +369,7 @@ def main():
         clocks.start()
         time.sleep(1.0)
     for _ in range(args.warmup):
-        _, radii, _ = step(prm)
+        color, radii, da = step(prm)
     barrier()
     V = int((radii > 0).sum())
     D = int(R.last_pair_count(dev))
@@ -375,7 +399,7 @@ def main():
     e0.record()
     marks[0].record()
     for i in range(args.steps):
-        step(prm)
+        color, radii, da = step(prm)
         marks[i + 1].record()
     e1.record()
     barrier()
@@ -384,6 +408,9 @@ def main():
     stages = _lib.profile_collect()
     _lib.profile_enable(0)
     R.flush_checks(dev)             # every forward's pair count has been checked against its capacity
+    dump = None
+    if args.dump_outputs and rank == 0:     # before grad_check and e2e overwrite the gradients
+        dump = dump_sample(color, radii, da, {**{k: prm[k].grad for k in names}, "means2D": m2d.grad}, P)
     t_ms = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
@@ -521,6 +548,10 @@ def main():
             line["reduce_mode"] = args.reduce if args.reduce != "backward" else f"backward/{args.sh_exchange}"
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_dict(wl, cpu_oracle_step(wl, 0))
+        if dump:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for k, v in dump.items():
+                np.save(os.path.join(args.dump_outputs, f"{k}.npy"), v)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

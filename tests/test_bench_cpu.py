@@ -29,3 +29,27 @@ def test_algorithmic_byte_model_matches_survey_magnitude():
     # sorted-record array, so it must come out lower but of the same magnitude
     assert 1.0e9 < total < 1.7e9
     assert alg["project_bwd"] > alg["project_sh"] and alg["scan_order"] == 0
+
+
+def test_dump_sample_is_seeded_typed_and_within_budget():
+    """--dump-outputs at the largest workload (1M Gaussians, 1024^2): float32/float64 only, at most 64 MB,
+    the same rows on every run, and every sampled row is the row of that Gaussian."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    P, H, W = 1_000_000, 1024, 1024
+    row = torch.arange(P, dtype=torch.float32)
+    grads = {k: row.reshape(P, *[1] * len(s)).expand(P, *s) for k, s in
+             (("means3D", (3,)), ("opacities", (1,)), ("shs", (16, 3)), ("scales", (3,)), ("rotations", (4,)), ("means2D", (3,)))}
+    a = bench.dump_sample(torch.zeros(3, H, W), torch.arange(P, dtype=torch.int32), torch.zeros(2, H, W), grads, P)
+    b = bench.dump_sample(torch.ones(3, H, W), torch.arange(P, dtype=torch.int32), torch.ones(2, H, W), grads, P)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert a["color"].shape == (3, H, W) and a["depth_alpha"].shape == (2, H, W)
+    idx = a["sample_index"]
+    assert np.array_equal(idx, b["sample_index"]) and len(np.unique(idx)) == len(idx) == bench.DUMP_ROWS
+    assert np.array_equal(a["radii"], idx.astype(np.float32))
+    for k, v in grads.items():
+        assert a[f"grad_{k}"].shape == (len(idx), *v.shape[1:])
+        assert np.array_equal(a[f"grad_{k}"].reshape(len(idx), -1)[:, 0], idx.astype(np.float32))

@@ -1,42 +1,20 @@
-"""The drop-in contract checked against the reference's OWN call sites (CPU, build container only:
-/root/reference does not exist on the GPU box, so the test skips there).
+"""The drop-in contract checked against DreamScene's OWN call sites (CPU).
 
-/root/reference/scene_gaussian.py constructs GaussianRasterizationSettings and calls the rasterizer by
+DreamScene's scene_gaussian.py constructs GaussianRasterizationSettings and calls the rasterizer by
 keyword in three renderers (score_render :586-646, scene_render :737-870, object_render :951-1021).
-The file cannot be imported here (omegaconf, e3nn, pytorch3d, ... are missing), so its AST is parsed and
+Its call sites were read from its AST by tests/golden/make_call_sites.py into ref_call_sites.json;
 every keyword it passes is checked against the signatures this package exports under the same import
 name, plus the way it unpacks the results."""
-import ast
 import inspect
+import json
 import os
 
-import pytest
-
-REF = "/root/reference/scene_gaussian.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present (GPU box)")
-
-
-def _calls():
-    tree = ast.parse(open(REF).read())
-    imports = [n for n in ast.walk(tree) if isinstance(n, ast.ImportFrom) and n.module == "diff_gaussian_rasterization"]
-    settings, ctor, call = [], [], []
-    for n in ast.walk(tree):
-        if not isinstance(n, ast.Call):
-            continue
-        f = n.func
-        name = f.id if isinstance(f, ast.Name) else (f.attr if isinstance(f, ast.Attribute) else None)
-        if name == "GaussianRasterizationSettings":
-            settings.append(n)
-        elif name == "GaussianRasterizer":
-            ctor.append(n)
-        elif name == "rasterizer":
-            call.append(n)
-    return imports, settings, ctor, call, tree
+SITES = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_call_sites.json")))
+SCENE = SITES["scene_gaussian.py"]
 
 
 def test_reference_imports_exactly_what_the_alias_package_exports():
-    imports, *_ = _calls()
-    names = sorted(a.name for n in imports for a in n.names)
+    names = sorted(SCENE["imports"])
     assert names == ["GaussianRasterizationSettings", "GaussianRasterizer"]
     import diff_gaussian_rasterization as D
     for n in names:
@@ -45,35 +23,29 @@ def test_reference_imports_exactly_what_the_alias_package_exports():
 
 def test_every_keyword_the_reference_passes_is_accepted():
     from diff_gaussian_rasterization import GaussianRasterizationSettings, GaussianRasterizer
-    _, settings, ctor, call, _ = _calls()
+    settings, ctor, call = SCENE["settings"], SCENE["ctor"], SCENE["call"]
     assert len(settings) == 3 and len(ctor) == 3 and len(call) == 3       # score / scene / object renderers
     fields = set(GaussianRasterizationSettings._fields)
     for n in settings:
-        assert not n.args, "settings are passed by keyword"
-        kws = {k.arg for k in n.keywords}
+        assert not n["n_args"], "settings are passed by keyword"
+        kws = set(n["keywords"])
         assert kws <= fields, kws - fields
         required = {f for f in GaussianRasterizationSettings._fields if f not in GaussianRasterizationSettings._field_defaults}
         assert required <= kws, required - kws
     init = inspect.signature(GaussianRasterizer.__init__)
     for n in ctor:
-        assert {k.arg for k in n.keywords} == {"raster_settings"} and "raster_settings" in init.parameters
+        assert set(n["keywords"]) == {"raster_settings"} and "raster_settings" in init.parameters
     fwd = inspect.signature(GaussianRasterizer.forward)
     for n in call:
-        assert not n.args
-        kws = {k.arg for k in n.keywords}
+        assert not n["n_args"]
+        kws = set(n["keywords"])
         assert kws == {"means3D", "means2D", "shs", "colors_precomp", "opacities", "scales", "rotations", "cov3D_precomp"}
         assert kws <= set(fwd.parameters)
 
 
 def test_result_unpacking_matches_the_return_arity():
     """score_render unpacks 4 values (important_score first), scene/object_render 3."""
-    *_, tree = _calls()
-    arities = []
-    for n in ast.walk(tree):
-        if isinstance(n, ast.Assign) and isinstance(n.value, ast.Call):
-            f = n.value.func
-            if isinstance(f, ast.Name) and f.id == "rasterizer" and isinstance(n.targets[0], ast.Tuple):
-                arities.append([getattr(e, "id", None) for e in n.targets[0].elts])
+    arities = [n["targets"] for n in SCENE["unpack"]]
     assert sorted(len(a) for a in arities) == [3, 3, 4]
     four = [a for a in arities if len(a) == 4][0]
     assert four[0] == "important_score" and four[1:] == ["rendered_image", "radii", "depth_alpha"]
@@ -84,11 +56,9 @@ def test_result_unpacking_matches_the_return_arity():
 
 def test_simple_knn_call_site():
     """gs_renderer.py:9 imports distCUDA2 from simple_knn._C and calls it with one positional tensor (:590-593)."""
-    src = "/root/reference/gs_renderer.py"
-    tree = ast.parse(open(src).read())
-    imp = [n for n in ast.walk(tree) if isinstance(n, ast.ImportFrom) and n.module == "simple_knn._C"]
-    assert imp and [a.name for a in imp[0].names] == ["distCUDA2"]
-    calls = [n for n in ast.walk(tree) if isinstance(n, ast.Call) and isinstance(n.func, ast.Name) and n.func.id == "distCUDA2"]
-    assert calls and all(len(c.args) == 1 and not c.keywords for c in calls)
+    knn = SITES["gs_renderer.py"]
+    assert knn["imports"] and knn["imports"][0] == ["distCUDA2"]
+    calls = knn["call"]
+    assert calls and all(c["n_args"] == 1 and not c["keywords"] for c in calls)
     from simple_knn._C import distCUDA2
     assert list(inspect.signature(distCUDA2).parameters) == ["points"]
