@@ -60,9 +60,8 @@ class ScratchLayout(C.Structure):
 
 
 _lib = None
-ABI_VERSION = 3
+ABI_VERSION = 4
 FWD_NO_BACKWARD = 1
-BWD_COMPOSITE, BWD_PROJECT = 1, 2
 
 
 def load():
@@ -92,7 +91,7 @@ def load():
         [vp, sz, vp, sz, u64, u32, vp, u32, vp]
     lib.b200gsr_backward.argtypes = [C.POINTER(Params)] + [vp] * 7 + [vp] * 4 + \
         [vp, sz, vp, sz, u64] + [vp] * 8 + [vp]
-    lib.b200gsr_backward_ex.argtypes = lib.b200gsr_backward.argtypes[:-1] + [u32, i32, i32, i32, vp]
+    lib.b200gsr_backward_ex.argtypes = lib.b200gsr_backward.argtypes[:-1] + [i32, vp]
     lib.b200gsr_backward_ex.restype = C.c_int
     lib.b200gsr_mark_visible.argtypes = [i32, vp, vp, vp, vp, vp]
     lib.b200gsr_sh_grad_expand.argtypes = [i32, i32, i32, i32, vp, vp, sz, vp, vp]

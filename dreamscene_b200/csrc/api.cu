@@ -246,13 +246,10 @@ int b200gsr_backward_ex(const b200gsr_params* prm, const float* means3D, const f
                      const float* dL_ddepth_alpha, void* saved, size_t saved_bytes,
                      void* /*scratch*/, size_t /*scratch_bytes*/, uint64_t max_pairs, float* d_means3D,
                      float* d_means2D, float* d_shs, float* d_colors, float* d_opacities,
-                     float* d_scales, float* d_rotations, float* d_cov3D, uint32_t stages,
-                     int32_t g_begin, int32_t g_end, int32_t dsh_coefs, void* stream) {
+                     float* d_scales, float* d_rotations, float* d_cov3D, int32_t dsh_coefs, void* stream) {
     int rc = validate_inputs(prm, means3D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp);
     if (rc) return rc;
     if (prm->P == 0) return B200GSR_OK;
-    if (g_begin < 0 || g_end > prm->P || g_begin > g_end || (g_begin % 128) != 0)
-        return fail(B200GSR_ERR_BAD_ARG, "bad Gaussian range [%d, %d): need 0 <= begin <= end <= P, begin %% 128 == 0", g_begin, g_end);
     if (shs && dsh_coefs != 0 && dsh_coefs != -1 &&
         (dsh_coefs < (prm->sh_degree + 1) * (prm->sh_degree + 1) || dsh_coefs > prm->M))
         return fail(B200GSR_ERR_BAD_ARG, "dsh_coefs=%d must be 0, -1 or in [(sh_degree+1)^2, M]", dsh_coefs);
@@ -280,32 +277,25 @@ int b200gsr_backward_ex(const b200gsr_params* prm, const float* means3D, const f
     a.d_means3D = d_means3D; a.d_means2D = d_means2D; a.d_shs = d_shs; a.d_colors = d_colors;
     a.d_opac = d_opacities; a.d_scales = d_scales; a.d_rots = d_rotations; a.d_cov3d = d_cov3D;
     a.num_sms = ds->num_sms; a.stats = g_stats;
-    a.g_begin = g_begin; a.g_end = g_end; a.dsh_coefs = dsh_coefs;
+    a.dsh_coefs = dsh_coefs;
     a.view = 0; a.num_views = 1; a.P_view = prm->P; a.gy_view = gsr_grid(prm->image_height, prm->image_width).gy;
     a.accumulate = 0;
     a.stream = static_cast<cudaStream_t>(stream);
 
     // no memsets: the work-queue counters and the gradient accumulators live in `saved`, zeroed by
     // the forward and restored to zero by project_bwd
-    const bool whole = (stages & B200GSR_BWD_COMPOSITE) && (stages & B200GSR_BWD_PROJECT) && g_begin == 0 && g_end == prm->P;
-    if (stages & B200GSR_BWD_COMPOSITE) {
-        if (whole) prof_mark_bwd(0, a.stream);
-        GSR_RANGE_PUSH("b200gsr.composite_bwd");
-        rc = check_cuda(gsr_launch_composite_bwd(a), "composite_bwd");
-        GSR_RANGE_POP();
-        if (rc) return rc;
-    }
-    if (stages & B200GSR_BWD_PROJECT) {
-        if (whole) prof_mark_bwd(1, a.stream);
-        GSR_RANGE_PUSH("b200gsr.project_bwd");
-        rc = check_cuda(gsr_launch_project_bwd(a), "project_bwd");
-        GSR_RANGE_POP();
-        if (rc) return rc;
-    }
-    if (whole) {
-        prof_mark_bwd(2, a.stream);
-        if (g_prof.max_calls > 0 && g_prof.nbwd < g_prof.max_calls) ++g_prof.nbwd;
-    }
+    prof_mark_bwd(0, a.stream);
+    GSR_RANGE_PUSH("b200gsr.composite_bwd");
+    rc = check_cuda(gsr_launch_composite_bwd(a), "composite_bwd");
+    GSR_RANGE_POP();
+    if (rc) return rc;
+    prof_mark_bwd(1, a.stream);
+    GSR_RANGE_PUSH("b200gsr.project_bwd");
+    rc = check_cuda(gsr_launch_project_bwd(a), "project_bwd");
+    GSR_RANGE_POP();
+    if (rc) return rc;
+    prof_mark_bwd(2, a.stream);
+    if (g_prof.max_calls > 0 && g_prof.nbwd < g_prof.max_calls) ++g_prof.nbwd;
     return B200GSR_OK;
 }
 
@@ -320,7 +310,7 @@ int b200gsr_backward(const b200gsr_params* prm, const float* means3D, const floa
     return b200gsr_backward_ex(prm, means3D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp, radii,
                                out_depth_alpha, dL_dcolor, dL_ddepth_alpha, saved, saved_bytes, scratch, scratch_bytes,
                                max_pairs, d_means3D, d_means2D, d_shs, d_colors, d_opacities, d_scales, d_rotations,
-                               d_cov3D, B200GSR_BWD_COMPOSITE | B200GSR_BWD_PROJECT, 0, prm ? prm->P : 0, 0, stream);
+                               d_cov3D, 0, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -428,7 +418,7 @@ int b200gsr_backward_views(int32_t B, const b200gsr_params* prm, const b200gsr_v
     a.radii = radii; a.out_depth_alpha = out_depth_alpha; a.dL_dcolor = dL_dcolor; a.dL_ddepth_alpha = dL_ddepth_alpha;
     a.saved = static_cast<uint8_t*>(saved); a.scratch = nullptr; a.max_pairs = (uint32_t)max_pairs;
     a.num_sms = ds->num_sms; a.stats = g_stats;
-    a.num_views = B; a.P_view = P; a.gy_view = g1.gy; a.dsh_coefs = 0; a.g_begin = 0; a.g_end = P;
+    a.num_views = B; a.P_view = P; a.gy_view = g1.gy; a.dsh_coefs = 0;
     a.stream = static_cast<cudaStream_t>(stream);
     a.prm = prm[0]; a.view = 0; a.accumulate = 0;
     a.means3D = in[0].means3D; a.shs = in[0].shs; a.colors = in[0].colors_precomp; a.opac = in[0].opacities;

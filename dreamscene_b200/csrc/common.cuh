@@ -136,22 +136,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 }
 #endif  // __CUDACC__
 
-#ifdef __CUDACC__
-// Fetch the next work item (index into the longest-first work order, < limit) from the split
-// queue; returns false when every sub-queue is exhausted.  Call from one thread.
-__device__ __forceinline__ bool gsr_queue_pop(uint32_t* counters, uint32_t limit, uint32_t& q, uint32_t& tried,
-                                              uint32_t& item) {
-    while (tried < GSR_NQUEUE) {
-        const uint32_t i = atomicAdd(counters + q, 1u);
-        const uint32_t w = i * GSR_NQUEUE + q;
-        if (w < limit) { item = w; return true; }
-        q = (q + 1) % GSR_NQUEUE;
-        ++tried;
-    }
-    return false;
-}
-#endif
-
 // ---- kernel launchers (defined in the .cu files, called from api.cu) ---------------------
 struct GsrFwdArgs {
     b200gsr_params prm;
@@ -187,7 +171,6 @@ struct GsrBwdArgs {
     float *d_means3D, *d_means2D, *d_shs, *d_colors, *d_opac, *d_scales, *d_rots, *d_cov3d;
     int view, num_views, P_view, gy_view;   // see GsrFwdArgs
     int accumulate;        // project_bwd adds into the gradient outputs instead of overwriting (views sharing a parameter)
-    int g_begin, g_end;    // Gaussian range of the project_bwd stage (chunked launches)
     int dsh_coefs;         // coefficients per row of d_shs (0 = M, the reference layout)
     int num_sms;
     unsigned long long* stats;   // optional device counters (b200gsr_debug_counters); selects the STATS kernels

@@ -19,10 +19,7 @@
 //   * backward: per-(warp, Gaussian) partial gradients are reduced with a halving shuffle
 //     butterfly (12 SHFL for 10 values) and committed with ONE coalesced RED instruction.
 #include "common.cuh"
-#include <cuda.h>          // CUtensorMap types only; the encoder is fetched with cudaGetDriverEntryPoint
 #include <cuda_fp16.h>
-#include <cstdlib>
-#include <cstring>
 
 namespace {
 
@@ -30,20 +27,10 @@ namespace {
 // ordered longest list first).  Every warp is an independent worker with a private ring of kSlots
 // sub-chunks (32 records = one per lane): the backward kernel contains no CTA-wide barrier.
 constexpr int kWarps = 8;      // warps per CTA (in the backward kernel just a container)
-#ifndef GSR_BWD_DEFAULT_VARIANT
-#define GSR_BWD_DEFAULT_VARIANT 10    // which backward kernel ships (see gsr_launch_composite_bwd)
-#endif
-#ifndef GSR_FWD_ILP
-#define GSR_FWD_ILP 2                 // list entries in flight per warp in the forward (A/B: B200GSR_FWD_VARIANT=51..54)
-#endif
-#ifndef GSR_BWD_KFAST
-#define GSR_BWD_KFAST 2               // fast-path width of the STATS instantiation
-#endif
-// kSlots (template parameter of the backward kernel) = sub-chunks in the ring per warp
-// (kSlots-1 being gathered + 1 being blended); 1.5 KB per slot and warp.
-template <int kSlots>
+constexpr int kSlots = 3;      // sub-chunks in the ring per warp (kSlots-1 being gathered + 1 being blended)
+constexpr int kMinCtas = 4;    // backward CTAs per SM
 struct __align__(128) SmemRing {
-    GsrRec rec[kWarps][kSlots][32];
+    GsrRec rec[kWarps][kSlots][32];   // 1.5 KB per slot and warp
 };
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
@@ -61,14 +48,6 @@ __device__ __forceinline__ void gather_record(GsrRec* rec, const GsrRec* __restr
     cp_async16(dst, src);
     cp_async16(dst + 16, src + 16);
     cp_async16(dst + 32, src + 32);
-}
-
-// lane 0 pops the next item from the split queue, the warp gets it by shuffle
-__device__ __forceinline__ uint32_t warp_pop(uint32_t* queue, uint32_t limit, uint32_t& q, uint32_t& tried,
-                                             int lane) {
-    uint32_t item = 0xffffffffu;
-    if (lane == 0) gsr_queue_pop(queue, limit, q, tried, item);
-    return __shfl_sync(0xffffffffu, item, 0);
 }
 
 // Forward epilogue: a block that blended at least one entry becomes a work item of the backward, filed under
@@ -137,19 +116,16 @@ __device__ __forceinline__ unsigned long long gsr_now_ns() {
 // Forward keeps the tile as the unit of work: blocks that never saturate (silhouettes, thin
 // regions) must scan the whole list, and sharing each gathered 256-entry chunk between the 8
 // warps of the tile makes that scan cheap (measured: 0.145 ms vs 0.170 ms for independent warps).
-#ifndef GSR_FWD_CHUNK
-#define GSR_FWD_CHUNK 256
-#endif
-constexpr int kChunk = GSR_FWD_CHUNK;   // list entries per pipeline stage (kChunk/256 per thread)
+constexpr int kChunk = 256;   // list entries per pipeline stage (kChunk/256 per thread)
 struct __align__(128) SmemCta {
     GsrRec rec[2][kChunk];   // 2 x 12 KB at kChunk = 256
     uint32_t work;           // broadcast slot for the tile queue
 };
 
-// PARTS = 1: one CTA of 8 warps per tile.  PARTS = 2 (A/B variant): a tile is rendered by two CTAs of 4 warps,
-// each taking an 16x8 half (both gather the whole list; fewer warps per barrier, twice as many barrier groups).
-template <bool SCORE, int PPL, bool STATS, int PARTS = 1, int ILP = 1>
-__global__ void __launch_bounds__(256 / PPL / PARTS)
+// One CTA of 256/PPL threads per tile; each warp renders an 8x(4*PPL)-pixel block.  Only PPL = 1 (one pixel
+// per lane) is instantiated: 2 pixels per lane lost in round 1.
+template <bool SCORE, int PPL, bool STATS>
+__global__ void __launch_bounds__(256 / PPL)
 composite_fwd_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, const uint32_t* __restrict__ header,
                      const uint32_t* __restrict__ work_order,
                      const uint32_t* __restrict__ tile_start,
@@ -158,7 +134,7 @@ composite_fwd_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, cons
                      float* __restrict__ out_color, float* __restrict__ out_depth_alpha,
                      uint32_t* __restrict__ n_contrib, float* __restrict__ score,
                      unsigned long long* __restrict__ stats, uint32_t* bwd_fill, uint32_t* bwd_items) {
-    constexpr int kThreads = 256 / PPL / PARTS;
+    constexpr int kThreads = 256 / PPL;
     unsigned int st_eval = 0, st_lanes = 0;
     unsigned long long st_t0 = 0, st_item_t0 = 0, st_max_item_ns = 0;
     if (STATS) st_t0 = gsr_now_ns();
@@ -180,9 +156,9 @@ composite_fwd_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, cons
         __syncthreads();
         const uint32_t w = sm.work;
         __syncthreads();   // everyone has read the slot before thread 0 may overwrite it
-        if (w >= (uint32_t)ntiles * PARTS) break;
-        const uint32_t tile = work_order[w / PARTS];
-        const int blk = (int)(w % PARTS) * (kThreads / 32) + wid;      // 8x(4*PPL)-pixel block of the tile this warp renders
+        if (w >= (uint32_t)ntiles) break;
+        const uint32_t tile = work_order[w];
+        const int blk = wid;      // 8x(4*PPL)-pixel block of the tile this warp renders
         uint32_t beg = tile_start[tile], end = tile_start[tile + 1];
         if (end > max_pairs) end = max_pairs;
         if (beg > end) beg = end;
@@ -287,39 +263,32 @@ composite_fwd_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, cons
                     mask &= mask - 1;
                     const float4* rp = sp + 3 * b;
                     const float4 q0 = rp[0], q1 = rp[1], q2 = rp[2];
-                    if (ILP >= 2) {
-                        // ILP passing entries per trip: the record loads and exponents of the later ones are
-                        // in flight while the first is evaluated (a warp issues in order, so this divides the
-                        // dependent LDS -> FMA -> EX2 latency paid per entry on the longest tile, which bounds
-                        // the kernel: profiles/r02_balance.md).  Same arithmetic and order per entry.
-                        int bb[ILP];
-                        float4 r0[ILP], r1[ILP], r2[ILP];
-                        bb[0] = b; r0[0] = q0; r1[0] = q1; r2[0] = q2;
-                        int have = 1;                                      // warp-uniform
+                    // Two passing entries per trip: the record loads and exponent of the second are in flight
+                    // while the first is evaluated (a warp issues in order, so this halves the dependent
+                    // LDS -> FMA -> EX2 latency paid per entry on the longest tile, which bounds the kernel:
+                    // profiles/r02_balance.md).  Same arithmetic and order per entry.
+                    int bb[2];
+                    float4 r0[2], r1[2], r2[2];
+                    bb[0] = b; r0[0] = q0; r1[0] = q1; r2[0] = q2;
+                    int have = 1;                                      // warp-uniform
 #pragma unroll
-                        for (int j = 1; j < ILP; ++j) {
-                            const bool more = mask != 0u;
-                            bb[j] = more ? __ffs(mask) - 1 : b;
-                            mask &= mask - 1;                              // 0 stays 0
-                            have += more ? 1 : 0;
-                            const float4* rj = sp + 3 * bb[j];
-                            r0[j] = rj[0]; r1[j] = rj[1]; r2[j] = rj[2];
-                        }
-                        PairEval ev[ILP][PPL];
-#pragma unroll
-                        for (int j = 0; j < ILP; ++j)
-#pragma unroll
-                            for (int q = 0; q < PPL; ++q)
-                                ev[j][q] = eval_pair(r0[j].x, r0[j].y, r0[j].w, r1[j].x, r1[j].y, r1[j].z, X, Y[q]);
-#pragma unroll
-                        for (int j = 0; j < ILP; ++j)
-                            if (j < have) blend(r1[j], r2[j], ev[j], bb[j]);
-                    } else {
-                        PairEval ea[PPL];
-#pragma unroll
-                        for (int q = 0; q < PPL; ++q) ea[q] = eval_pair(q0.x, q0.y, q0.w, q1.x, q1.y, q1.z, X, Y[q]);
-                        blend(q1, q2, ea, b);
+                    for (int j = 1; j < 2; ++j) {
+                        const bool more = mask != 0u;
+                        bb[j] = more ? __ffs(mask) - 1 : b;
+                        mask &= mask - 1;                              // 0 stays 0
+                        have += more ? 1 : 0;
+                        const float4* rj = sp + 3 * bb[j];
+                        r0[j] = rj[0]; r1[j] = rj[1]; r2[j] = rj[2];
                     }
+                    PairEval ev[2][PPL];
+#pragma unroll
+                    for (int j = 0; j < 2; ++j)
+#pragma unroll
+                        for (int q = 0; q < PPL; ++q)
+                            ev[j][q] = eval_pair(r0[j].x, r0[j].y, r0[j].w, r1[j].x, r1[j].y, r1[j].z, X, Y[q]);
+#pragma unroll
+                    for (int j = 0; j < 2; ++j)
+                        if (j < have) blend(r1[j], r2[j], ev[j], bb[j]);
                 }
                 all_done = true;
 #pragma unroll
@@ -364,230 +333,16 @@ composite_fwd_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, cons
 }
 
 // =============================================================================================
-// Forward, Blackwell bulk-copy staging variants (A/B experiment for the north star's
-// "TMA/cp.async.bulk staging of per-tile Gaussian blocks"; profiles/r02_tma_ab.md):
-//   FWD_VARIANT 1: the tile's KEY chunks are staged with cp.async.bulk (UBLKCP) + mbarrier into a
-//                  3-deep shared-memory ring by one elected thread; records still move with LDGSTS;
-//   FWD_VARIANT 2: additionally the RECORDS are fetched with Blackwell's row-gather TMA,
-//                  cp.async.bulk.tensor.2d...tile::gather4 over geom viewed as f32[P][12]: one
-//                  instruction per 4 records (64 per chunk) instead of 768 LDGSTS.
-// Key chunks start at an arbitrary pair offset (8-byte granularity); bulk copies need 16-byte
-// aligned sources, so the copy starts at the even pair index at or below the chunk start and is
-// two keys longer (the key array has two spare entries at its end for exactly this).
+// Backward.  The kernel is called composite_bwd2 because it replaced round 1's composite_bwd;
+// the profiling tools and the records in profiles/ know it by that name.  Per-(warp, Gaussian) body:
+//   * branch-free: non-contributing lanes run the same arithmetic with alpha = G = 0 instead of a
+//     divergent block + ten zero-initialisations (BSSY/BSYNC, 8 moves gone);
+//   * packed fp32 (fma.rn.f32x2 / mul / add -> FFMA2, FMUL2, FADD2): the four channel-parallel
+//     streams (r, g, b, depth) and the (x, y) geometry pairs go two per instruction, halving the
+//     fma-pipe occupancy of the body (the fma pipe retires a 3-register FFMA every 2 cycles/SMSP);
+//   * STATS instantiation counts evaluated / contributing (warp, Gaussian) pairs and the popcount
+//     histogram for the secondary (pair-evaluation) roofline in bench.py; never timed.
 // =============================================================================================
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE_%=;\n\t"
-        "bra WAIT_%=;\n\t"
-        "DONE_%=:\n\t}" :: "r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_gather4(void* dst, const void* tmap, int col, int r0, int r1, int r2, int r3,
-                                            unsigned long long* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes "
-                 "[%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
-                 :: "r"(smem_u32(dst)), "l"(tmap), "r"(col), "r"(r0), "r"(r1), "r"(r2), "r"(r3), "r"(smem_u32(bar))
-                 : "memory");
-}
-
-struct __align__(128) TmaMap { unsigned char bytes[128]; };   // CUtensorMap (opaque here)
-
-constexpr int kQuadF4 = 16;     // VARIANT 2: 4 records (12 float4) padded to 256 B so every gather4 lands 128-B aligned
-struct __align__(128) SmemFwdTma {
-    float4 rec[2][kChunk * 4];                       // VARIANT 1 uses [kChunk*3] of it (48-B records)
-    unsigned long long keys[3][kChunk + 2];
-    unsigned long long kbar[3];
-    unsigned long long rbar[2];
-    uint32_t work;
-};
-
-template <int VARIANT>
-__global__ void __launch_bounds__(256)
-composite_fwd_tma_kernel(int H, int W, int gx, int ntiles, const uint32_t* __restrict__ header,
-                         const uint32_t* __restrict__ work_order,
-                         const uint32_t* __restrict__ tile_start,
-                         const unsigned long long* __restrict__ keys, const GsrRec* __restrict__ geom,
-                         const __grid_constant__ TmaMap tmap,
-                         const float* __restrict__ bg, uint32_t* __restrict__ queue,
-                         float* __restrict__ out_color, float* __restrict__ out_depth_alpha,
-                         uint32_t* __restrict__ n_contrib, uint32_t* bwd_fill, uint32_t* bwd_items) {
-    constexpr int kThreads = 256;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    SmemFwdTma& sm = *reinterpret_cast<SmemFwdTma*>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const uint32_t max_pairs = header[GSR_H_MAX_PAIRS];
-    const float bg0 = __ldg(bg), bg1 = __ldg(bg + 1), bg2 = __ldg(bg + 2);
-    if (tid == 0) {
-        for (int i = 0; i < 3; ++i) mbar_init(&sm.kbar[i], 1);
-        for (int i = 0; i < 2; ++i) mbar_init(&sm.rbar[i], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t kphase = 0, rphase = 0;    // bit i = parity of the NEXT completion to wait for on barrier i
-
-    for (;;) {
-        if (tid == 0) sm.work = atomicAdd(queue, 1u);
-        __syncthreads();
-        const uint32_t w = sm.work;
-        __syncthreads();
-        if (w >= (uint32_t)ntiles) break;
-        const uint32_t tile = work_order[w];
-        uint32_t beg = tile_start[tile], end = tile_start[tile + 1];
-        if (end > max_pairs) end = max_pairs;
-        if (beg > end) beg = end;
-        const int n = (int)(end - beg);
-        const int nchunks = (n + kChunk - 1) / kChunk;
-        const int odd = (int)(beg & 1u);                       // 16-B alignment slack of this tile's key range
-        const unsigned long long* tk16 = keys + (beg - odd);   // even pair index: 16-byte aligned
-        const int tyi = tile / gx, txi = tile - tyi * gx;
-        const int X0i = txi * GSR_TILE + (wid & 1) * 8, Y0i = tyi * GSR_TILE + (wid >> 1) * 4;
-        const int Xi = X0i + (lane & 7), Yi = Y0i + (lane >> 3);
-        const float X0 = (float)X0i, Y0 = (float)Y0i, X = (float)Xi, Y = (float)Yi;
-        const bool inside = Xi < W && Yi < H;
-        bool done = !inside;
-        float T = 1.0f, Cr = 0.f, Cg = 0.f, Cb = 0.f, Dacc = 0.f;
-        uint32_t last = 0;
-
-        // issue the bulk copy of key chunk c into ring slot c % 3 (one elected thread)
-        auto issue_keys = [&](int c) {
-            if (tid == 0 && c < nchunks) {
-                const uint32_t bytes = (uint32_t)((kChunk + 2) * sizeof(unsigned long long));
-                mbar_expect_tx(&sm.kbar[c % 3], bytes);
-                bulk_g2s(sm.keys[c % 3], tk16 + (size_t)c * kChunk, bytes, &sm.kbar[c % 3]);
-            }
-        };
-        auto wait_keys = [&](int c) {
-            mbar_wait(&sm.kbar[c % 3], (kphase >> (c % 3)) & 1u);
-            kphase ^= 1u << (c % 3);
-        };
-        // gather the records of chunk c (keys already in shared memory) into record buffer c & 1
-        auto issue_records = [&](int c) {
-            const int cnt = min(kChunk, n - c * kChunk);
-            const unsigned long long* sk = sm.keys[c % 3] + odd;
-            if (VARIANT == 2) {
-                const int nq = (cnt + 3) >> 2;
-                if (tid == 0) mbar_expect_tx(&sm.rbar[c & 1], (uint32_t)nq * 4u * 48u);
-                __syncwarp();
-                if (tid < nq) {
-                    int r[4];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) r[j] = (4 * tid + j < cnt) ? (int)(uint32_t)sk[4 * tid + j] : 0;
-                    tma_gather4(&sm.rec[c & 1][tid * kQuadF4], &tmap, 0, r[0], r[1], r[2], r[3], &sm.rbar[c & 1]);
-                }
-            } else {
-                if (tid < cnt) gather_record(reinterpret_cast<GsrRec*>(sm.rec[c & 1]) + tid, geom, sk[tid]);
-                cp_async_commit();
-            }
-        };
-        auto wait_records = [&](int c) {
-            if (VARIANT == 2) {
-                mbar_wait(&sm.rbar[c & 1], (rphase >> (c & 1)) & 1u);
-                rphase ^= 1u << (c & 1);
-            } else {
-                cp_async_wait<0>();
-            }
-        };
-
-        int keys_issued = 0, keys_waited = 0, recs_issued = 0, recs_waited = 0;
-        if (nchunks > 0) {
-            issue_keys(0); issue_keys(1); keys_issued = min(2, nchunks);
-            wait_keys(0); keys_waited = 1;
-            issue_records(0); recs_issued = 1;
-        }
-        for (int c = 0; c < nchunks; ++c) {
-            wait_records(c); recs_waited = c + 1;
-            // everyone's view of chunk c is complete, everyone is done with chunk c-1 (its record buffer
-            // and the key slot (c+2) % 3 == (c-1) % 3 are free); doubles as the CTA-wide early-out vote
-            const int ndone = __syncthreads_count(done);
-            if (ndone == kThreads) break;
-            if (c + 2 < nchunks) { issue_keys(c + 2); keys_issued = c + 3; }
-            if (c + 1 < nchunks) {
-                wait_keys(c + 1); keys_waited = c + 2;
-                issue_records(c + 1); recs_issued = c + 2;
-            }
-            const int cnt = min(kChunk, n - c * kChunk);
-            if (__all_sync(0xffffffffu, done)) continue;   // this warp is saturated
-            for (int sub = 0; sub * 32 < cnt; ++sub) {
-                const int r = sub * 32 + lane;
-                bool pass = false;
-                if (r < cnt) {
-                    const float4 q0 = (VARIANT == 2) ? sm.rec[c & 1][(r >> 2) * kQuadF4 + (r & 3) * 3] : sm.rec[c & 1][3 * r];
-                    pass = cull_pass(q0.x, q0.y, __float_as_uint(q0.z), X0, Y0);
-                }
-                uint32_t mask = __ballot_sync(0xffffffffu, pass);
-                const uint32_t pos0 = (uint32_t)(c * kChunk + sub * 32 + 1);
-                while (mask) {
-                    const int b = __ffs(mask) - 1;
-                    mask &= mask - 1;
-                    const int e = sub * 32 + b;
-                    const float4* rp = (VARIANT == 2) ? &sm.rec[c & 1][(e >> 2) * kQuadF4 + (e & 3) * 3] : &sm.rec[c & 1][3 * e];
-                    const float4 q0 = rp[0], q1 = rp[1], q2 = rp[2];
-                    const PairEval ev = eval_pair(q0.x, q0.y, q0.w, q1.x, q1.y, q1.z, X, Y);
-                    if (ev.valid && !done) {
-                        const float Tn = T * (1.0f - ev.alpha);
-                        if (Tn < GSR_T_STOP) {
-                            done = true;
-                        } else {
-                            const float wgt = ev.alpha * T;
-                            Cr = fmaf(q2.x, wgt, Cr); Cg = fmaf(q2.y, wgt, Cg); Cb = fmaf(q2.z, wgt, Cb);
-                            Dacc = fmaf(q1.w, wgt, Dacc);
-                            T = Tn;
-                            last = pos0 + (uint32_t)b;
-                        }
-                    }
-                }
-                if (__all_sync(0xffffffffu, done)) break;
-            }
-        }
-        // never leave bulk copies in flight across tiles (early-out case): drain what was issued
-        while (recs_waited < recs_issued) { wait_records(recs_waited); ++recs_waited; }
-        while (keys_waited < keys_issued) { wait_keys(keys_waited); ++keys_waited; }
-        __syncthreads();
-
-        if (inside) {
-            const size_t plane = (size_t)H * W;
-            const size_t pix = (size_t)Yi * W + Xi;
-            out_color[pix] = fmaf(T, bg0, Cr);
-            out_color[plane + pix] = fmaf(T, bg1, Cg);
-            out_color[2 * plane + pix] = fmaf(T, bg2, Cb);
-            out_depth_alpha[pix] = Dacc;
-            out_depth_alpha[plane + pix] = T;
-            n_contrib[pix] = last;
-        }
-        const uint32_t nb = __reduce_max_sync(0xffffffffu, last);
-        if ((tid & 31) == 0) bwd_item_append(bwd_fill, bwd_items, ntiles, tile, tid >> 5, nb);
-    }
-}
-
-// =============================================================================================
-// Backward
-// =============================================================================================
-// Halving butterfly: after the call v[0] of lane L holds the warp-wide sum of value
-// `vidx(L)` (see bwd_value_index); 5+3+2+1+1 = 12 shuffles for 10 values.
-template <int N, int XOR>
-__device__ __forceinline__ void halve(float (&v)[10], bool hi) {
-    constexpr int Hh = (N + 1) / 2;
-#pragma unroll
-    for (int k = 0; k < Hh; ++k) {
-        const float lo = v[k];
-        const float hv = (Hh + k < N) ? v[Hh + k] : 0.0f;
-        const float send = hi ? lo : hv;
-        const float keep = hi ? hv : lo;
-        v[k] = keep + __shfl_xor_sync(0xffffffffu, send, XOR);
-    }
-}
 __device__ __forceinline__ int bwd_value_index(int lane) {
     // which of the 10 values this lane ends up owning (-1: a padding slot)
     int base = 0, n = 10;
@@ -598,172 +353,9 @@ __device__ __forceinline__ int bwd_value_index(int lane) {
     return n >= 1 ? base : -1;
 }
 
-template <int kSlots, int kMinCtas>
-__global__ void __launch_bounds__(kWarps * 32, kMinCtas)
-composite_bwd_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, const uint32_t* __restrict__ header,
-                     const uint32_t* __restrict__ work_order,
-                     const uint32_t* __restrict__ tile_start,
-                     const unsigned long long* __restrict__ keys, const GsrRec* __restrict__ geom,
-                     const float* __restrict__ bg, uint32_t* __restrict__ queue,
-                     const float* __restrict__ out_depth_alpha,
-                     const uint32_t* __restrict__ n_contrib, const float* __restrict__ dL_dcolor,
-                     const float* __restrict__ dL_ddepth_alpha, float* __restrict__ dgeom) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    SmemRing<kSlots>& sm = *reinterpret_cast<SmemRing<kSlots>*>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    GsrRec (*ring)[32] = sm.rec[wid];
-    const uint32_t max_pairs = header[GSR_H_MAX_PAIRS];
-    const uint32_t nonempty = header[GSR_H_NUM_NONEMPTY];
-    const int vidx = bwd_value_index(lane);
-    const bool commit_lane = (vidx >= 0) && !(lane & 1);
-    const size_t plane = (size_t)Hs * W;
-
-    uint32_t qsel = (blockIdx.x * kWarps + wid) % GSR_NQUEUE, qtried = 0;
-    for (;;) {
-        const uint32_t item = warp_pop(queue, nonempty * 8u, qsel, qtried, lane);   // empty tiles: no gradient
-        if (item == 0xffffffffu) break;
-        const uint32_t tile = work_order[item >> 3];
-        const int blk = (int)(item & 7u);
-        uint32_t beg = tile_start[tile], end = tile_start[tile + 1];
-        if (end > max_pairs) end = max_pairs;
-        if (beg > end) beg = end;
-        const unsigned long long* tk = keys + beg;
-        const int tys = tile / gx, txi = tile - tys * gx;
-        const int view = tys / gy_view, tyi = tys - view * gy_view;      // view-local evaluation, stacked addressing
-        const int row0 = view * gy_view * GSR_TILE;
-        const float* bgv = bg + 3 * view;
-        const float bg0 = __ldg(bgv), bg1 = __ldg(bgv + 1), bg2 = __ldg(bgv + 2);
-        const int X0i = txi * GSR_TILE + (blk & 1) * 8, Y0i = tyi * GSR_TILE + (blk >> 1) * 4;
-        const int Xi = X0i + (lane & 7), Yi = Y0i + (lane >> 3);
-        const float X0 = (float)X0i, Y0 = (float)Y0i, X = (float)Xi, Y = (float)Yi;
-        uint32_t last = 0;
-        float Tfinal = 1.f, dC0 = 0.f, dC1 = 0.f, dC2 = 0.f, dD = 0.f, dT = 0.f;
-        if (Xi < W && Yi < H) {
-            const size_t pix = (size_t)(row0 + Yi) * W + Xi;
-            last = n_contrib[pix];
-            Tfinal = out_depth_alpha[plane + pix];
-            dC0 = dL_dcolor[pix]; dC1 = dL_dcolor[plane + pix]; dC2 = dL_dcolor[2 * plane + pix];
-            dD = dL_ddepth_alpha[pix]; dT = dL_ddepth_alpha[plane + pix];
-        }
-        if ((int)last > (int)(end - beg)) last = end - beg;   // overflow safety
-        const int n = (int)__reduce_max_sync(0xffffffffu, last);   // only entries [0, n) reached this block
-        const int nsub = (n + 31) >> 5;
-        const float bgterm = bg0 * dC0 + bg1 * dC1 + bg2 * dC2 + dT;
-        float T = Tfinal, accR = 0.f, accG = 0.f, accB = 0.f, accD = 0.f;
-
-        // sub-chunks are visited from the back: visit v <-> sub-chunk nsub-1-v
-        unsigned long long kq0, kq1;
-        {
-            unsigned long long kk[kSlots + 1];
-#pragma unroll
-            for (int j = 0; j < kSlots + 1; ++j) {
-                const int e = (nsub - 1 - j) * 32 + lane;
-                kk[j] = (j < nsub && e < n) ? __ldg(tk + e) : 0ull;
-            }
-#pragma unroll
-            for (int j = 0; j < kSlots - 1; ++j) {
-                const int e = (nsub - 1 - j) * 32 + lane;
-                if (j < nsub && e < n) gather_record(&ring[j][lane], geom, kk[j]);
-                cp_async_commit();
-            }
-            kq0 = kk[kSlots - 1]; kq1 = kk[kSlots];
-        }
-        for (int v = 0; v < nsub; ++v) {
-            {
-                const int g = v + kSlots - 1;
-                if (g < nsub) gather_record(&ring[g % kSlots][lane], geom, kq0);   // earlier sub-chunks are full
-                cp_async_commit();
-                kq0 = kq1;
-                const int g2 = v + kSlots + 1;
-                kq1 = (g2 < nsub) ? __ldg(tk + (nsub - 1 - g2) * 32 + lane) : 0ull;
-            }
-            cp_async_wait<kSlots - 1>();
-            __syncwarp();
-            const GsrRec* st = ring[v % kSlots];
-            const int sidx = nsub - 1 - v;
-            const int cnt = min(32, n - sidx * 32);
-            bool pass = false;
-            if (lane < cnt) {
-                const float4 q0 = *reinterpret_cast<const float4*>(&st[lane]);
-                pass = cull_pass(q0.x, q0.y, __float_as_uint(q0.z), X0, Y0);
-            }
-            uint32_t mask = __ballot_sync(0xffffffffu, pass);
-            const float4* sp = reinterpret_cast<const float4*>(st);
-            const uint32_t pos0 = (uint32_t)(sidx * 32 + 1);
-            while (mask) {
-                const int b = 31 - __clz(mask);
-                mask &= ~(1u << b);
-                const float4* rp = sp + 3 * b;
-                const float4 q0 = rp[0], q1 = rp[1], q2 = rp[2];
-                const uint32_t pos = pos0 + (uint32_t)b;
-                const PairEval e = eval_pair(q0.x, q0.y, q0.w, q1.x, q1.y, q1.z, X, Y);
-                const bool contrib = e.valid && pos <= last;
-                if (!__any_sync(0xffffffffu, contrib)) continue;
-                float vv[10];
-#pragma unroll
-                for (int j = 0; j < 10; ++j) vv[j] = 0.f;
-                if (contrib) {
-                    const float om = 1.0f - e.alpha;
-                    const float rom = rcp_approx(om);
-                    T = T * rom;                       // transmittance in front of this entry
-                    const float wgt = e.alpha * T;
-                    float dLda = (q2.x - accR) * dC0 + (q2.y - accG) * dC1 + (q2.z - accB) * dC2 +
-                                 (q1.w - accD) * dD;
-                    dLda = dLda * T - (Tfinal * rom) * bgterm;
-                    accR = fmaf(e.alpha, q2.x - accR, accR);
-                    accG = fmaf(e.alpha, q2.y - accG, accG);
-                    accB = fmaf(e.alpha, q2.z - accB, accB);
-                    accD = fmaf(e.alpha, q1.w - accD, accD);
-                    const float gG = q1.z * dLda * e.G;   // dL/dG * G (no zeroing under the 0.99 clamp)
-#ifdef GSR_EXACT_EXP
-                    const float gxs = -(q0.w * e.dx + q1.x * e.dy);    // d ln G / d px, raw conic
-                    const float gys = -(q1.y * e.dy + q1.x * e.dx);
-#else
-                    const float gxs = 2.0f * q0.w * e.dx + q1.x * e.dy;
-                    const float gys = 2.0f * q1.y * e.dy + q1.x * e.dx;
-#endif
-                    vv[0] = gG * gxs; vv[1] = gG * gys;
-                    vv[2] = gG * e.dx * e.dx; vv[3] = gG * e.dx * e.dy; vv[4] = gG * e.dy * e.dy;
-                    vv[5] = e.G * dLda;
-                    vv[6] = wgt * dC0; vv[7] = wgt * dC1; vv[8] = wgt * dC2; vv[9] = wgt * dD;
-                }
-                halve<10, 16>(vv, lane & 16);
-                halve<5, 8>(vv, lane & 8);
-                halve<3, 4>(vv, lane & 4);
-                halve<2, 2>(vv, lane & 2);
-                const float tot = vv[0] + __shfl_xor_sync(0xffffffffu, vv[0], 1);
-                if (commit_lane) atomicAdd(dgeom + 12 * (size_t)__float_as_uint(q2.w) + vidx, tot);
-            }
-            __syncwarp();
-        }
-        cp_async_wait<0>();
-        __syncwarp();
-    }
-}
-
-
-// ---------------------------------------------------------------------------------------------
-// Backward, round-2 variant ("v2"): same work decomposition and ring as composite_bwd_kernel, with an
-// instruction diet on the per-(warp, Gaussian) body (VERDICT r1 item 2):
-//   * branch-free: non-contributing lanes run the same arithmetic with alpha = G = 0 instead of a
-//     divergent block + ten zero-initialisations (BSSY/BSYNC, 8 moves gone);
-//   * packed fp32 (fma.rn.f32x2 / mul / add -> FFMA2, FMUL2, FADD2): the four channel-parallel
-//     streams (r, g, b, depth) and the (x, y) geometry pairs go two per instruction, halving the
-//     fma-pipe occupancy of the body (the fma pipe retires a 3-register FFMA every 2 cycles/SMSP);
-//   * small-footprint fast path: when at most KFAST lanes of the warp contribute, those lanes commit
-//     their ten partials directly with three vector reductions (red.global.add.v4.f32, sm_90+:
-//     dgeom rows are 3 x 16 B) instead of the 12-shuffle butterfly;
-//   * STATS instantiation counts evaluated / contributing (warp, Gaussian) pairs and the popcount
-//     histogram for the secondary (pair-evaluation) roofline in bench.py; never timed.
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" :: "l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
-__device__ __forceinline__ void red_add_v2(float* addr, float a, float b) {
-    asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" :: "l"(addr), "f"(a), "f"(b) : "memory");
-}
-
-// packed halving step on float2 pairs is not possible (selects are per register), but the ADDs are
+// Halving butterfly: after the four calls and one last shuffle, lane L holds the warp-wide sum of value
+// `vidx(L)` (see bwd_value_index); 5+3+2+1+1 = 12 shuffles for 10 values.  The selects are per register,
+// the ADDs go in packed pairs.
 template <int N, int XOR>
 __device__ __forceinline__ void halve2(float (&v)[10], bool hi) {
     constexpr int Hh = (N + 1) / 2;
@@ -785,7 +377,7 @@ __device__ __forceinline__ void halve2(float (&v)[10], bool hi) {
 }
 
 
-template <int kSlots, int kMinCtas, int KFAST, bool STATS, bool DUAL = false>
+template <bool STATS>
 __global__ void __launch_bounds__(kWarps * 32, kMinCtas)
 composite_bwd2_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, const uint32_t* __restrict__ header,
                       const uint32_t* __restrict__ work_order,
@@ -797,7 +389,7 @@ composite_bwd2_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, con
                       const float* __restrict__ dL_ddepth_alpha, float* __restrict__ dgeom,
                       unsigned long long* __restrict__ stats, const uint32_t* __restrict__ bwd_items) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    SmemRing<kSlots>& sm = *reinterpret_cast<SmemRing<kSlots>*>(smem_raw);
+    SmemRing& sm = *reinterpret_cast<SmemRing*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     GsrRec (*ring)[32] = sm.rec[wid];
     const uint32_t max_pairs = header[GSR_H_MAX_PAIRS];
@@ -924,101 +516,6 @@ composite_bwd2_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, con
             uint32_t mask = __ballot_sync(0xffffffffu, pass);
             const float4* sp = reinterpret_cast<const float4*>(st);
             const uint32_t pos0 = (uint32_t)(sidx * 32 + 1);
-#ifndef GSR_EXACT_EXP
-            if (DUAL) {
-                // Two passing entries per trip.  A warp issues in order, so with one entry per trip every
-                // dependent step (LDS -> FMA -> EX2 -> ballot -> body -> 5 shuffle levels) is paid in full per
-                // entry; the longest (tile, block) item - a serial chain of several hundred entries - bounds the
-                // kernel (profiles/r02_balance.md).  Here both entries' loads, exponents and butterflies are
-                // independent instruction streams the scheduler interleaves; only the T / accumulated-colour
-                // recurrences stay serial.  Per-entry arithmetic and decisions are unchanged.
-                auto alpha_of = [&](const float4& q0, const float4& q1, float2& d, float& G, float& alpha) {
-                    d = __fadd2_rn(make_float2(q0.x, q0.y), XY);
-                    const float u = __fmaf_rn(q0.w, d.x, __fmul_rn(q1.x, d.y));
-                    const float p2 = __fmaf_rn(__fmul_rn(q1.y, d.y), d.y, __fmul_rn(u, d.x));
-                    G = ex2_approx(p2);
-                    alpha = fminf(GSR_ALPHA_MAX, __fmul_rn(q1.z, G));
-                    return (p2 <= 0.0f) && (alpha >= GSR_ALPHA_MIN);
-                };
-                auto body = [&](const float4& q0, const float4& q1, const float4& q2, const float2& d, float G,
-                                float alpha, bool contrib, float (&vv)[10]) {
-                    const float am = contrib ? alpha : 0.0f;
-                    const float Gm = contrib ? G : 0.0f;
-                    const float rom = rcp_approx(1.0f - am);
-                    T = contrib ? T * rom : T;
-                    const float wgt = am * T;
-                    const float2 c01 = make_float2(q2.x, q2.y), c2D = make_float2(q2.z, q1.w);
-                    const float2 d01 = __fadd2_rn(c01, make_float2(-acc01.x, -acc01.y));
-                    const float2 d2D = __fadd2_rn(c2D, make_float2(-acc2D.x, -acc2D.y));
-                    const float2 dot2 = __ffma2_rn(d2D, dC2D, __fmul2_rn(d01, dC01));
-                    const float dLda = (dot2.x + dot2.y) * T - bgT * rom;
-                    const float2 am2 = make_float2(am, am);
-                    acc01 = __ffma2_rn(am2, d01, acc01);
-                    acc2D = __ffma2_rn(am2, d2D, acc2D);
-                    vv[5] = Gm * dLda;
-                    const float gG = q1.z * vv[5];
-                    const float2 gs = __ffma2_rn(make_float2(q0.w + q0.w, q1.y + q1.y), d,
-                                                 __fmul2_rn(make_float2(q1.x, q1.x), make_float2(d.y, d.x)));
-                    const float2 gG2 = make_float2(gG, gG);
-                    const float2 v01 = __fmul2_rn(gG2, gs);
-                    const float2 tu = __fmul2_rn(gG2, d);
-                    const float2 v24 = __fmul2_rn(tu, d);
-                    vv[0] = v01.x; vv[1] = v01.y; vv[2] = v24.x; vv[3] = tu.x * d.y; vv[4] = v24.y;
-                    const float2 w2 = make_float2(wgt, wgt);
-                    const float2 v67 = __fmul2_rn(w2, dC01), v89 = __fmul2_rn(w2, dC2D);
-                    vv[6] = v67.x; vv[7] = v67.y; vv[8] = v89.x; vv[9] = v89.y;
-                };
-                while (mask) {
-                    const int b0 = 31 - __clz(mask);
-                    mask &= ~(1u << b0);
-                    const bool two = mask != 0u;                          // warp-uniform
-                    const int b1 = two ? 31 - __clz(mask) : b0;
-                    mask &= ~(1u << b1);
-                    const float4* rpa = sp + 3 * b0;
-                    const float4* rpb = sp + 3 * b1;
-                    const float4 a0 = rpa[0], a1 = rpa[1], c0 = rpb[0], c1 = rpb[1];
-                    float2 da, db;
-                    float Ga, Gb, alpa, alpb;
-                    const bool va = alpha_of(a0, a1, da, Ga, alpa);
-                    const bool vb = alpha_of(c0, c1, db, Gb, alpb);
-                    const bool ca = va && (pos0 + (uint32_t)b0) <= last;
-                    const bool cb = two && vb && (pos0 + (uint32_t)b1) <= last;
-                    const uint32_t cma = __ballot_sync(0xffffffffu, ca);
-                    const uint32_t cmb = __ballot_sync(0xffffffffu, cb);
-                    if ((cma | cmb) == 0u) continue;
-                    float wa[10], wb[10];
-                    float *rowa = dgeom, *rowb = dgeom;
-                    if (cma != 0u) {
-                        const float4 a2 = rpa[2];
-                        body(a0, a1, a2, da, Ga, alpa, ca, wa);
-                        rowa = dgeom + 12 * (size_t)__float_as_uint(a2.w);
-                    }
-                    if (cmb != 0u) {
-                        const float4 c2 = rpb[2];
-                        body(c0, c1, c2, db, Gb, alpb, cb, wb);
-                        rowb = dgeom + 12 * (size_t)__float_as_uint(c2.w);
-                    }
-                    if (cma != 0u && cmb != 0u) {
-                        halve2<10, 16>(wa, lane & 16); halve2<10, 16>(wb, lane & 16);
-                        halve2<5, 8>(wa, lane & 8);    halve2<5, 8>(wb, lane & 8);
-                        halve2<3, 4>(wa, lane & 4);    halve2<3, 4>(wb, lane & 4);
-                        halve2<2, 2>(wa, lane & 2);    halve2<2, 2>(wb, lane & 2);
-                        const float ta = wa[0] + __shfl_xor_sync(0xffffffffu, wa[0], 1);
-                        const float tb = wb[0] + __shfl_xor_sync(0xffffffffu, wb[0], 1);
-                        if (commit_lane) { atomicAdd(rowa + vidx, ta); atomicAdd(rowb + vidx, tb); }
-                    } else {
-                        float (&w1)[10] = cma != 0u ? wa : wb;
-                        float* row1 = cma != 0u ? rowa : rowb;
-                        halve2<10, 16>(w1, lane & 16);
-                        halve2<5, 8>(w1, lane & 8);
-                        halve2<3, 4>(w1, lane & 4);
-                        halve2<2, 2>(w1, lane & 2);
-                        const float t1 = w1[0] + __shfl_xor_sync(0xffffffffu, w1[0], 1);
-                        if (commit_lane) atomicAdd(row1 + vidx, t1);
-                    }
-                }
-            } else
-#endif
             while (mask) {
                 const int b = 31 - __clz(mask);
                 mask &= ~(1u << b);
@@ -1074,18 +571,10 @@ composite_bwd2_kernel(int H, int W, int gx, int gy_view, int Hs, int ntiles, con
                 const float2 v67 = __fmul2_rn(w2, dC01), v89 = __fmul2_rn(w2, dC2D);
                 vv[6] = v67.x; vv[7] = v67.y; vv[8] = v89.x; vv[9] = v89.y;
                 float* row = dgeom + 12 * (size_t)__float_as_uint(q2.w);
-                const int k = __popc(cm);
                 if (STATS) {
+                    const int k = __popc(cm);
                     ++st_contrib; st_lanes += k;
                     ++st_hist[k == 1 ? 0 : k == 2 ? 1 : k <= 4 ? 2 : k <= 8 ? 3 : k <= 16 ? 4 : 5];
-                }
-                if (KFAST > 0 && k <= KFAST) {
-                    if (contrib) {
-                        red_add_v4(row, vv[0], vv[1], vv[2], vv[3]);
-                        red_add_v4(row + 4, vv[4], vv[5], vv[6], vv[7]);
-                        red_add_v2(row + 8, vv[8], vv[9]);
-                    }
-                    continue;
                 }
                 halve2<10, 16>(vv, lane & 16);
                 halve2<5, 8>(vv, lane & 8);
@@ -1145,54 +634,15 @@ static CompPtrs comp_ptrs(const uint8_t* saved, const b200gsr_saved_layout& vl, 
     return c;
 }
 
-template <bool SCORE, bool STATS, int ILP = 1>
+template <bool SCORE, bool STATS>
 static cudaError_t launch_fwd(const GsrFwdArgs& a, int nblocks, const CompPtrs& c, uint32_t* queue) {
     const int smem = (int)sizeof(SmemCta);
     static std::atomic<unsigned long long> attr_done{0};
-    cudaError_t e = gsr_smem_once(composite_fwd_kernel<SCORE, 1, STATS, 1, ILP>, smem, attr_done);
+    cudaError_t e = gsr_smem_once(composite_fwd_kernel<SCORE, 1, STATS>, smem, attr_done);
     if (e != cudaSuccess) return e;
-    composite_fwd_kernel<SCORE, 1, STATS, 1, ILP><<<nblocks, 256, smem, a.stream>>>(
+    composite_fwd_kernel<SCORE, 1, STATS><<<nblocks, 256, smem, a.stream>>>(
         a.prm.image_height, a.prm.image_width, c.grid.gx, a.gy_view, c.H, c.grid.ntiles, c.header, c.work_order, c.tile_start,
         c.keys, c.geom, a.prm.bg, queue, a.out_color, a.out_depth_alpha, c.n_contrib, a.score, a.stats, c.bwd_fill, c.bwd_items);
-    return cudaGetLastError();
-}
-
-// ---- tensor map for the gather4 variant: geom viewed as f32[P][12], box = one 48-byte row ------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static cudaError_t make_geom_tensor_map(const GsrRec* geom, int P, TmaMap* out) {
-    static EncodeTiledFn encode = [] {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess ||
-            q != cudaDriverEntryPointSuccess) fn = nullptr;
-        return reinterpret_cast<EncodeTiledFn>(fn);
-    }();
-    if (!encode) return cudaErrorNotSupported;
-    static_assert(sizeof(CUtensorMap) == sizeof(TmaMap), "tensor map size");
-    const cuuint64_t dims[2] = {12, (cuuint64_t)(P > 0 ? P : 1)};
-    const cuuint64_t strides[1] = {sizeof(GsrRec)};
-    const cuuint32_t box[2] = {12, 1};
-    const cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(reinterpret_cast<CUtensorMap*>(out), CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
-                        const_cast<GsrRec*>(geom), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? cudaSuccess : cudaErrorInvalidValue;
-}
-
-template <int VARIANT>
-static cudaError_t launch_fwd_tma(const GsrFwdArgs& a, int nblocks, const CompPtrs& c, uint32_t* queue) {
-    const int smem = (int)sizeof(SmemFwdTma);
-    static std::atomic<unsigned long long> attr_done{0};
-    cudaError_t e = gsr_smem_once(composite_fwd_tma_kernel<VARIANT>, smem, attr_done);
-    if (e != cudaSuccess) return e;
-    TmaMap tmap;
-    memset(&tmap, 0, sizeof(tmap));
-    if (VARIANT == 2 && (e = make_geom_tensor_map(c.geom, a.prm.P, &tmap)) != cudaSuccess) return e;
-    composite_fwd_tma_kernel<VARIANT><<<nblocks, 256, smem, a.stream>>>(
-        a.prm.image_height, a.prm.image_width, c.grid.gx, c.grid.ntiles, c.header, c.work_order, c.tile_start,
-        c.keys, c.geom, tmap, a.prm.bg, queue, a.out_color, a.out_depth_alpha, c.n_contrib, c.bwd_fill, c.bwd_items);
     return cudaGetLastError();
 }
 
@@ -1201,76 +651,21 @@ cudaError_t gsr_launch_composite_fwd(const GsrFwdArgs& a) {
     if (c.grid.ntiles == 0) return cudaSuccess;
     uint32_t* queue = reinterpret_cast<uint32_t*>(a.scratch + a.sl.counters) + GSR_C_FWD_QUEUE;
     const int nblocks = min(c.grid.ntiles, a.num_sms * 6);
-    // B200GSR_FWD_VARIANT = 1 | 2: bulk-copy / TMA staging experiments (profiles/r02_tma_ab.md)
-    static const int fwd_variant = [] { const char* e = getenv("B200GSR_FWD_VARIANT"); return e ? atoi(e) : 0; }();
-    if (fwd_variant >= 51 && fwd_variant <= 54 && !a.prm.score_flag && a.stats == nullptr) {   // 1/2/3/4 list entries in flight
-        return fwd_variant == 51 ? launch_fwd<false, false, 1>(a, nblocks, c, queue)
-             : fwd_variant == 52 ? launch_fwd<false, false, 2>(a, nblocks, c, queue)
-             : fwd_variant == 53 ? launch_fwd<false, false, 3>(a, nblocks, c, queue)
-                                 : launch_fwd<false, false, 4>(a, nblocks, c, queue);
-    }
-    if ((fwd_variant == 42 || fwd_variant == 44) && !a.prm.score_flag && a.stats == nullptr) {
-        // a tile rendered by 2 (4) CTAs of 4 (2) warps, two entries in flight: finer work items for the balance
-        const int smem = (int)sizeof(SmemCta);
-        static std::atomic<unsigned long long> attr_done42{0}, attr_done44{0};
-        if (fwd_variant == 42) {
-            cudaError_t e4 = gsr_smem_once(composite_fwd_kernel<false, 1, false, 2, 2>, smem, attr_done42);
-            if (e4 != cudaSuccess) return e4;
-            composite_fwd_kernel<false, 1, false, 2, 2><<<min(2 * c.grid.ntiles, a.num_sms * 8), 128, smem, a.stream>>>(
-                a.prm.image_height, a.prm.image_width, c.grid.gx, a.gy_view, c.H, c.grid.ntiles, c.header, c.work_order, c.tile_start,
-                c.keys, c.geom, a.prm.bg, queue, a.out_color, a.out_depth_alpha, c.n_contrib, a.score, a.stats, c.bwd_fill, c.bwd_items);
-        } else {
-            cudaError_t e4 = gsr_smem_once(composite_fwd_kernel<false, 1, false, 4, 2>, smem, attr_done44);
-            if (e4 != cudaSuccess) return e4;
-            composite_fwd_kernel<false, 1, false, 4, 2><<<min(4 * c.grid.ntiles, a.num_sms * 9), 64, smem, a.stream>>>(
-                a.prm.image_height, a.prm.image_width, c.grid.gx, a.gy_view, c.H, c.grid.ntiles, c.header, c.work_order, c.tile_start,
-                c.keys, c.geom, a.prm.bg, queue, a.out_color, a.out_depth_alpha, c.n_contrib, a.score, a.stats, c.bwd_fill, c.bwd_items);
-        }
-        return cudaGetLastError();
-    }
-    if (fwd_variant == 4 && !a.prm.score_flag && a.stats == nullptr) {     // two 4-warp CTAs per tile
-        const int smem = (int)sizeof(SmemCta);
-        static std::atomic<unsigned long long> attr_done4{0};
-        cudaError_t e4 = gsr_smem_once(composite_fwd_kernel<false, 1, false, 2>, smem, attr_done4);
-        if (e4 != cudaSuccess) return e4;
-        const int nb4 = min(2 * c.grid.ntiles, a.num_sms * 8);
-        composite_fwd_kernel<false, 1, false, 2><<<nb4, 128, smem, a.stream>>>(
-            a.prm.image_height, a.prm.image_width, c.grid.gx, a.gy_view, c.H, c.grid.ntiles, c.header, c.work_order, c.tile_start,
-            c.keys, c.geom, a.prm.bg, queue, a.out_color, a.out_depth_alpha, c.n_contrib, a.score, a.stats, c.bwd_fill, c.bwd_items);
-        return cudaGetLastError();
-    }
-    if (fwd_variant != 0 && !a.prm.score_flag && a.stats == nullptr && a.num_views == 1) {
-        const int nb = min(c.grid.ntiles, a.num_sms * 5);
-        return fwd_variant == 2 ? launch_fwd_tma<2>(a, nb, c, queue) : launch_fwd_tma<1>(a, nb, c, queue);
-    }
     if (a.stats != nullptr)
-        return a.prm.score_flag ? launch_fwd<true, true, GSR_FWD_ILP>(a, nblocks, c, queue)
-                                : launch_fwd<false, true, GSR_FWD_ILP>(a, nblocks, c, queue);
-    return a.prm.score_flag ? launch_fwd<true, false, GSR_FWD_ILP>(a, nblocks, c, queue)
-                            : launch_fwd<false, false, GSR_FWD_ILP>(a, nblocks, c, queue);
+        return a.prm.score_flag ? launch_fwd<true, true>(a, nblocks, c, queue)
+                                : launch_fwd<false, true>(a, nblocks, c, queue);
+    return a.prm.score_flag ? launch_fwd<true, false>(a, nblocks, c, queue)
+                            : launch_fwd<false, false>(a, nblocks, c, queue);
 }
 
-template <int kSlots, int kMinCtas>
+template <bool STATS>
 static cudaError_t launch_bwd(const GsrBwdArgs& a, const CompPtrs& c, uint32_t* queue, float* dgeom) {
-    const int smem = (int)sizeof(SmemRing<kSlots>);
+    const int smem = (int)sizeof(SmemRing);
     const int nblocks = min(c.grid.ntiles, a.num_sms * kMinCtas);
     static std::atomic<unsigned long long> attr_done{0};
-    cudaError_t e = gsr_smem_once(composite_bwd_kernel<kSlots, kMinCtas>, smem, attr_done);
+    cudaError_t e = gsr_smem_once(composite_bwd2_kernel<STATS>, smem, attr_done);
     if (e != cudaSuccess) return e;
-    composite_bwd_kernel<kSlots, kMinCtas><<<nblocks, kWarps * 32, smem, a.stream>>>(
-        a.prm.image_height, a.prm.image_width, c.grid.gx, a.gy_view, c.H, c.grid.ntiles, c.header, c.work_order, c.tile_start,
-        c.keys, c.geom, a.prm.bg, queue, a.out_depth_alpha, c.n_contrib, a.dL_dcolor, a.dL_ddepth_alpha, dgeom);
-    return cudaGetLastError();
-}
-
-template <int kSlots, int kMinCtas, int KFAST, bool STATS, bool DUAL = false>
-static cudaError_t launch_bwd2(const GsrBwdArgs& a, const CompPtrs& c, uint32_t* queue, float* dgeom) {
-    const int smem = (int)sizeof(SmemRing<kSlots>);
-    const int nblocks = min(c.grid.ntiles, a.num_sms * kMinCtas);
-    static std::atomic<unsigned long long> attr_done{0};
-    cudaError_t e = gsr_smem_once(composite_bwd2_kernel<kSlots, kMinCtas, KFAST, STATS, DUAL>, smem, attr_done);
-    if (e != cudaSuccess) return e;
-    composite_bwd2_kernel<kSlots, kMinCtas, KFAST, STATS, DUAL><<<nblocks, kWarps * 32, smem, a.stream>>>(
+    composite_bwd2_kernel<STATS><<<nblocks, kWarps * 32, smem, a.stream>>>(
         a.prm.image_height, a.prm.image_width, c.grid.gx, a.gy_view, c.H, c.grid.ntiles, c.header, c.work_order, c.tile_start,
         c.keys, c.geom, a.prm.bg, queue, a.out_depth_alpha, c.n_contrib, a.dL_dcolor, a.dL_ddepth_alpha, dgeom,
         a.stats, c.bwd_items);
@@ -1282,28 +677,5 @@ cudaError_t gsr_launch_composite_bwd(const GsrBwdArgs& a) {
     if (c.grid.ntiles == 0) return cudaSuccess;
     uint32_t* queue = reinterpret_cast<uint32_t*>(a.saved + a.vl.header) + GSR_H_BWD_QUEUE;
     float* dgeom = reinterpret_cast<float*>(a.saved + a.vl.dgeom);
-    if (a.stats != nullptr) return launch_bwd2<3, 4, GSR_BWD_KFAST, true>(a, c, queue, dgeom);
-    // B200GSR_BWD_VARIANT selects kernels for A/B runs (profiles/r02_bwd_ab.md): 0 = round-1 kernel,
-    // 10/11/12/14 = v2 with the direct-commit fast path for <= 0/1/2/4 contributing lanes;
-    // B200GSR_BWD_SLOTS = ring depth x CTAs/SM of the round-1 kernel (tuned default 3 x 4)
-    static const int variant = [] { const char* e = getenv("B200GSR_BWD_VARIANT"); return e ? atoi(e) : GSR_BWD_DEFAULT_VARIANT; }();
-    switch (variant) {
-        case 10: return launch_bwd2<3, 4, 0, false>(a, c, queue, dgeom);
-        case 11: return launch_bwd2<3, 4, 1, false>(a, c, queue, dgeom);
-        case 12: return launch_bwd2<3, 4, 2, false>(a, c, queue, dgeom);
-        case 14: return launch_bwd2<3, 4, 4, false>(a, c, queue, dgeom);
-        case 125: return launch_bwd2<3, 5, 2, false>(a, c, queue, dgeom);
-        case 30: return launch_bwd2<3, 4, 0, false, true>(a, c, queue, dgeom);     // two entries in flight per warp, 64 registers
-        case 33: return launch_bwd2<3, 3, 0, false, true>(a, c, queue, dgeom);     // ... 3 CTAs/SM (85 registers)
-        case 32: return launch_bwd2<3, 2, 0, false, true>(a, c, queue, dgeom);     // ... 2 CTAs/SM (128 registers)
-        default: break;
-    }
-    static const int slots = [] { const char* e = getenv("B200GSR_BWD_SLOTS"); return e ? atoi(e) : 3; }();
-    switch (slots) {
-        case 2: return launch_bwd<2, 4>(a, c, queue, dgeom);
-        case 25: return launch_bwd<2, 5>(a, c, queue, dgeom);
-        case 35: return launch_bwd<3, 5>(a, c, queue, dgeom);
-        case 4: return launch_bwd<4, 4>(a, c, queue, dgeom);
-        default: return launch_bwd<3, 4>(a, c, queue, dgeom);
-    }
+    return a.stats != nullptr ? launch_bwd<true>(a, c, queue, dgeom) : launch_bwd<false>(a, c, queue, dgeom);
 }

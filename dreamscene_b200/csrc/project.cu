@@ -10,7 +10,6 @@
 // written in the oracle, so those integers are bit-exact against it.
 #include "common.cuh"
 #include <cuda_fp16.h>
-#include <cstdlib>
 
 #define MUL(a, b) __fmul_rn((a), (b))
 #define ADD(a, b) __fadd_rn((a), (b))
@@ -421,8 +420,11 @@ project_sh_kernel(b200gsr_params p, const float* __restrict__ means3D,
 //   2: sum g*dx*dx  3: sum g*dx*dy  4: sum g*dy*dy
 //   5: sum G*dL/dalpha (dL/dopacity)   6..8: dL/drgb   9: dL/ddepth   10,11: unused
 // =========================================================================================
-template <int MT, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB)
+// Register budget: since the parameter loads were hoisted above the SH wait (they overlap the cp.async
+// staging), 8 CTAs/SM (64 registers) spills: measured 0.147 ms vs 0.120 ms at 6 CTAs/SM (80 registers)
+// and 0.142 ms before the overlap.
+template <int MT>
+__global__ void __launch_bounds__(kBlock, 6)
 project_bwd_kernel(b200gsr_params p, const float* __restrict__ means3D,
                    const float* __restrict__ shs, const float* __restrict__ colors,
                    const float* __restrict__ scales, const float* __restrict__ rots,
@@ -435,8 +437,7 @@ project_bwd_kernel(b200gsr_params p, const float* __restrict__ means3D,
                    float* __restrict__ d_rots, float* __restrict__ d_cov3d) {
     extern __shared__ __align__(16) float sh_buf[];
     __shared__ uint8_t vis_s[kBlock];
-    // this launch covers Gaussians [g_base, g_end) (the whole range, or one chunk when the host
-    // overlaps the gradient all-reduce of finished chunks with the remaining ones)
+    // this launch covers Gaussians [g_base, g_end); the launcher passes the whole view [0, P_view)
     const int g0 = g_base + blockIdx.x * kBlock;
     const int i = g0 + threadIdx.x;
     const bool active = i < g_end;
@@ -786,38 +787,23 @@ cudaError_t gsr_launch_project(const GsrFwdArgs& a) {
     return cudaGetLastError();
 }
 
-template <int MT, int MINB>
-static void launch_project_bwd_v(const GsrBwdArgs& a, int g_begin, int g_end, size_t smem) {
-    project_bwd_kernel<MT, MINB><<<(g_end - g_begin + kBlock - 1) / kBlock, kBlock, smem, a.stream>>>(
+template <int MT>
+static void launch_project_bwd(const GsrBwdArgs& a, size_t smem) {
+    project_bwd_kernel<MT><<<(a.P_view + kBlock - 1) / kBlock, kBlock, smem, a.stream>>>(
         a.prm, a.means3D, a.shs, a.colors, a.scales, a.rots, a.cov3d, a.radii,
         reinterpret_cast<float*>(a.saved + a.vl.dgeom),
-        reinterpret_cast<uint32_t*>(a.saved + a.vl.header) + GSR_H_BWD_QUEUE, g_begin, g_end,
+        reinterpret_cast<uint32_t*>(a.saved + a.vl.header) + GSR_H_BWD_QUEUE, 0, a.P_view,
         a.dsh_coefs > 0 ? a.dsh_coefs : (a.dsh_coefs < 0 ? -1 : a.prm.M), a.view * a.P_view, a.accumulate, a.d_means3D,
         a.d_means2D, a.d_shs,
         a.d_colors, a.d_opac, a.d_scales, a.d_rots, a.d_cov3d);
 }
 
-// register budget of project_bwd.  Since the parameter loads were hoisted above the SH wait (they overlap the
-// cp.async staging), 8 CTAs/SM (64 registers) spills: measured 0.147 ms vs 0.120 ms at 6 CTAs/SM (80 registers)
-// and 0.142 ms before the overlap.  B200GSR_PBWD_MINB = 8 | 6 | 5 selects for A/B runs.
-#ifndef GSR_PBWD_DEFAULT_MINB
-#define GSR_PBWD_DEFAULT_MINB 6
-#endif
-template <int MT>
-static void launch_project_bwd(const GsrBwdArgs& a, int g_begin, int g_end, size_t smem) {
-    static const int minb = [] { const char* e = getenv("B200GSR_PBWD_MINB"); return e ? atoi(e) : GSR_PBWD_DEFAULT_MINB; }();
-    if (minb == 8) launch_project_bwd_v<MT, 8>(a, g_begin, g_end, smem);
-    else if (minb == 5) launch_project_bwd_v<MT, 5>(a, g_begin, g_end, smem);
-    else launch_project_bwd_v<MT, 6>(a, g_begin, g_end, smem);
-}
-
 cudaError_t gsr_launch_project_bwd(const GsrBwdArgs& a) {
-    const int g_begin = a.g_begin, g_end = a.g_end;
-    if (g_end <= g_begin) return cudaSuccess;
+    if (a.P_view <= 0) return cudaSuccess;
     const size_t smem = a.shs ? (size_t)kBlock * sh_row_stride(a.prm.M) * sizeof(float) : 0;
-    if (a.shs && a.prm.M == 16) launch_project_bwd<16>(a, g_begin, g_end, smem);
-    else if (a.shs && a.prm.M == 4) launch_project_bwd<4>(a, g_begin, g_end, smem);
-    else launch_project_bwd<0>(a, g_begin, g_end, smem);
+    if (a.shs && a.prm.M == 16) launch_project_bwd<16>(a, smem);
+    else if (a.shs && a.prm.M == 4) launch_project_bwd<4>(a, smem);
+    else launch_project_bwd<0>(a, smem);
     return cudaGetLastError();
 }
 

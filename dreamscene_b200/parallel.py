@@ -15,10 +15,10 @@ are summed over NCCL/NVLink.  Two ways to do the sum, both additive to the refer
 
 2. ``enable_view_sharding(mode="backward")``: the rasterizer's backward all-reduces its flat
    parameter-gradient buffer itself (ONE ncclAllReduce, no staging copy) and sends only the active
-   degree's SH columns.  ``chunks=K > 1`` pipelines the reduction over K Gaussian ranges, overlapping
-   finished chunks with the per-Gaussian backward of the rest; measured on 4 x B200 this LOSES
-   (1.82 vs 1.44 ms/step at K=8: 40 small collectives cost more than the 0.14 ms of project_bwd they
-   can hide; profiles/r02_scale_probe.md), so the default is K=1.
+   degree's SH columns.  Pipelining that reduction over Gaussian ranges, overlapping finished ranges
+   with the per-Gaussian backward of the rest, was measured on 4 x B200 to lose (1.82 vs 1.44 ms/step
+   at 8 ranges: 40 small collectives cost more than the 0.14 ms of project_bwd they can hide;
+   profiles/r02_scale_probe.md).
    By default the SH gradient is not all-reduced at all: dL/dsh of a view is basis(view direction) x
    dL/dcolour, so the ranks all-gather 3 floats per Gaussian (+ their camera centre) and rebuild the summed
    [P, M, 3] rows locally (``exchange_factored``; sh_exchange="dense" restores the row all-reduce).
@@ -36,35 +36,33 @@ from __future__ import annotations
 
 import contextlib
 import os
-from typing import Iterable, Optional, Sequence
+from typing import Iterable, Optional
 
 import torch
 import torch.distributed as dist
 
 _group = None
 _enabled = False
-_chunks = 1
 _sh_exchange = "factored"
 _suspended = 0
 MAX_FACTORED_VIEWS = 64          # b200gsr_sh_grad_expand
 _CHECK = bool(int(os.environ.get("B200GSR_CHECK_COLLECTIVES", "0")))
 
 
-def enable_view_sharding(group: Optional["dist.ProcessGroup"] = None, mode: str = "backward", chunks: int = 1,
+def enable_view_sharding(group: Optional["dist.ProcessGroup"] = None, mode: str = "backward",
                          sh_exchange: str = "factored") -> None:
     """mode="backward": every rasterizer backward all-reduces its parameter gradients (see the module
     docstring for when that is exact); mode="deferred": nothing happens inside backward, call
-    all_reduce_gradients() yourself.  `chunks` = number of Gaussian ranges the in-backward
-    reduction is pipelined over.  sh_exchange="factored" (default, chunks == 1, SH inputs): the SH gradient
+    all_reduce_gradients() yourself.  sh_exchange="factored" (default, SH inputs): the SH gradient
     is exchanged as 3 floats per Gaussian and view and rebuilt on every rank; "dense": all-reduced as rows."""
-    global _group, _enabled, _chunks, _sh_exchange
+    global _group, _enabled, _sh_exchange
     if not dist.is_initialized():
         raise RuntimeError("torch.distributed is not initialised")
     if mode not in ("backward", "deferred"):
         raise ValueError("mode must be 'backward' or 'deferred'")
     if sh_exchange not in ("factored", "dense"):
         raise ValueError("sh_exchange must be 'factored' or 'dense'")
-    _group, _enabled, _chunks, _sh_exchange = group, mode == "backward", max(1, int(chunks)), sh_exchange
+    _group, _enabled, _sh_exchange = group, mode == "backward", sh_exchange
 
 
 def disable_view_sharding() -> None:
@@ -93,7 +91,7 @@ def reduction_active() -> bool:
 
 def factored_sh_exchange() -> bool:
     """The in-backward reduction sends the SH gradient in factored form (see exchange_factored)."""
-    return (reduction_active() and _sh_exchange == "factored" and _chunks <= 1
+    return (reduction_active() and _sh_exchange == "factored"
             and dist.get_world_size(_group) <= MAX_FACTORED_VIEWS)
 
 
@@ -133,32 +131,16 @@ def exchange_factored(flat: torch.Tensor, dcol: torch.Tensor, P: int, M: int, sh
     return d_sh
 
 
-def chunk_bounds(P: int, chunks: Optional[int] = None, align: int = 128):
-    """Split [0, P) into <= chunks ranges whose starts are multiples of `align`."""
-    chunks = _chunks if chunks is None else chunks
-    if P <= 0:
-        return []
-    per = -(-P // chunks)
-    per = max(align, -(-per // align) * align)
-    return [(g, min(P, g + per)) for g in range(0, P, per)]
-
-
-def _coalesced_all_reduce(tensors, group, async_ops: bool):
+def _coalesced_all_reduce(tensors, group):
     """One NCCL group call for all tensors (ncclGroupStart/End); plain per-tensor calls on backends
-    without coalescing support (gloo in the CPU tests).  Returns an object with .wait()."""
+    without coalescing support (gloo in the CPU tests).  Returns when the sums are in place."""
     if dist.get_backend(group) == "nccl":
-        with dist._coalescing_manager(group=group, device=tensors[0].device, async_ops=async_ops) as cm:
+        with dist._coalescing_manager(group=group, device=tensors[0].device, async_ops=False):
             for t in tensors:
                 dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
-        return cm
-    works = [dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group, async_op=async_ops) for t in tensors]
-
-    class _Works:
-        def wait(self):
-            for w in works:
-                if w is not None:
-                    w.wait()
-    return _Works()
+        return
+    for t in tensors:
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
 
 
 def _check_same_size(numel: int, device="cuda") -> None:
@@ -169,28 +151,8 @@ def _check_same_size(numel: int, device="cuda") -> None:
                            f"max {int(t[0])}, min {-int(t[1])}): every rank must render the same P")
 
 
-class ChunkReducer:
-    """Issues one coalesced, asynchronous all-reduce per finished chunk (NCCL runs it on its own
-    stream after the kernels enqueued so far; the next chunk's kernel overlaps it)."""
-
-    def __init__(self, flat_numel: int, device="cuda"):
-        if _CHECK:
-            _check_same_size(flat_numel, device)
-        self.works = []
-
-    def reduce(self, pieces: Sequence[torch.Tensor]) -> None:
-        pieces = [p for p in pieces if p.numel() > 0]
-        if pieces:
-            self.works.append(_coalesced_all_reduce(pieces, _group, async_ops=True))
-
-    def wait(self) -> None:
-        for w in self.works:
-            w.wait()
-        self.works = []
-
-
 def maybe_all_reduce(flat: torch.Tensor) -> None:
-    """Monolithic reduction of a flat buffer (used when chunking does not apply)."""
+    """One all-reduce of a flat gradient buffer, when the in-backward reduction is active."""
     if reduction_active():
         if _CHECK:
             _check_same_size(flat.numel(), flat.device)
@@ -230,7 +192,7 @@ def all_reduce_gradients(params: Iterable[torch.Tensor], group: Optional["dist.P
         dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
         torch._foreach_copy_([t.reshape(-1) for t in tensors], list(flat.split([t.numel() for t in tensors])))
     else:
-        _coalesced_all_reduce(tensors, group, async_ops=False)
+        _coalesced_all_reduce(tensors, group)
     for dst, t in jobs:
         if dst is not None:
             dst.copy_(t)

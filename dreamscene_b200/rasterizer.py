@@ -402,9 +402,9 @@ class _RasterizeGaussians(torch.autograd.Function):
         g_da = torch.zeros(2, H, W, device=dev) if g_da is None else _f32c(g_da)
 
         # one flat buffer for every parameter gradient.  Under view sharding (dreamscene_b200.parallel,
-        # mode "backward") it is all-reduced chunk by chunk while later chunks are still being computed,
-        # and the SH section holds only the active degree's coefficients (the payload at sh_degree 0 is
-        # 14 instead of 59 floats per Gaussian); otherwise it is simply one allocation.
+        # mode "backward") it is all-reduced in one call after the backward kernels, and the SH section
+        # holds only the active degree's coefficients (the payload at sh_degree 0 is 14 instead of 59
+        # floats per Gaussian); otherwise it is simply one allocation.
         reduce = P > 0 and _parallel.reduction_active()
         ncoef = (int(rs.sh_degree) + 1) ** 2
         # factored: the SH gradient leaves the kernel as dL/dcolour [P, 3] and is exchanged by all-gather
@@ -414,7 +414,7 @@ class _RasterizeGaussians(torch.autograd.Function):
         offs, o = grad_sections(P, n_col, has_sr)
         flat = torch.empty(max(o, 1), dtype=torch.float32, device=dev)
         widths = {"means3D": 3, "opac": 1, "col": n_col, "scales": 3, "rots": 4, "cov": 6}
-        sec = lambda name, g0=0, g1=P: flat[offs[name] + g0 * widths[name]:offs[name] + g1 * widths[name]]
+        sec = lambda name: flat[offs[name]:offs[name] + P * widths[name]]
         d_means3D = sec("means3D").view(P, 3)
         d_opac = sec("opac").view(P, 1)
         d_colsh = sec("col")
@@ -442,35 +442,20 @@ class _RasterizeGaussians(torch.autograd.Function):
                 prm = st.prm
                 stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
-                def launch(stages, g0, g1):
-                    rc = lib.b200gsr_backward_ex(
-                        C.byref(prm), _ptr(means3D), _ptr(sh), _ptr(colors), _ptr(opacities), _ptr(scales),
-                        _ptr(rots), _ptr(cov3d), _ptr(radii), _ptr(depth_alpha), _ptr(g_color), _ptr(g_da),
-                        _ptr(st.saved), st.saved.numel(), None, 0, st.capacity,
-                        _ptr(d_means3D), _ptr(d_means2D), _ptr(d_sh), _ptr(d_colors), _ptr(d_opac),
-                        _ptr(d_scales), _ptr(d_rots), _ptr(d_cov), stages, g0, g1,
-                        -1 if factored else (ncoef if compact else 0), stream)
-                    if rc:
-                        raise RuntimeError(f"b200gsr_backward failed ({rc}): {_lib.last_error()}")
-
-                bounds = _parallel.chunk_bounds(P) if reduce else []
-                if not reduce:
-                    launch(_lib.BWD_COMPOSITE | _lib.BWD_PROJECT, 0, P)
-                elif factored:
-                    launch(_lib.BWD_COMPOSITE | _lib.BWD_PROJECT, 0, P)
+                rc = lib.b200gsr_backward_ex(
+                    C.byref(prm), _ptr(means3D), _ptr(sh), _ptr(colors), _ptr(opacities), _ptr(scales),
+                    _ptr(rots), _ptr(cov3d), _ptr(radii), _ptr(depth_alpha), _ptr(g_color), _ptr(g_da),
+                    _ptr(st.saved), st.saved.numel(), None, 0, st.capacity,
+                    _ptr(d_means3D), _ptr(d_means2D), _ptr(d_sh), _ptr(d_colors), _ptr(d_opac),
+                    _ptr(d_scales), _ptr(d_rots), _ptr(d_cov),
+                    -1 if factored else (ncoef if compact else 0), stream)
+                if rc:
+                    raise RuntimeError(f"b200gsr_backward failed ({rc}): {_lib.last_error()}")
+                if factored:
                     d_sh[3 * P:3 * P + 3].copy_(_const(rs.campos, dev).reshape(3))
                     d_sh = _parallel.exchange_factored(flat[:o], d_sh, P, M, int(rs.sh_degree), means3D)
-                elif len(bounds) <= 1:
-                    launch(_lib.BWD_COMPOSITE | _lib.BWD_PROJECT, 0, P)
+                elif reduce:
                     _parallel.maybe_all_reduce(flat[:o] if o > 0 else flat)      # ONE ncclAllReduce of the flat buffer
-                else:
-                    red = _parallel.ChunkReducer(flat.numel(), dev)
-                    launch(_lib.BWD_COMPOSITE, 0, 0)
-                    names = [k for k in ("means3D", "opac", "col", "scales", "rots", "cov") if k in offs]
-                    for g0, g1 in bounds:
-                        launch(_lib.BWD_PROJECT, g0, g1)
-                        red.reduce([sec(k, g0, g1) for k in names])
-                    red.wait()
             if compact:                      # expand to the reference layout [P, M, 3] (zeros above the degree)
                 full = torch.zeros(P, M, 3, dtype=torch.float32, device=dev)
                 full[:, :ncoef] = d_sh

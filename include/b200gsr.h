@@ -41,7 +41,7 @@
 extern "C" {
 #endif
 
-#define B200GSR_VERSION 3
+#define B200GSR_VERSION 4
 
 /* error codes */
 #define B200GSR_OK 0
@@ -158,14 +158,8 @@ int b200gsr_backward(const b200gsr_params* prm,
                      void* stream);
 
 /*
- * Staged / chunked backward (additive; no upstream equivalent).  Same arguments as
+ * Backward with a choice of SH gradient layout (additive; no upstream equivalent).  Same arguments as
  * b200gsr_backward plus
- *   stages    : B200GSR_BWD_COMPOSITE (per-pixel replay -> screen-space accumulators in `saved`)
- *               and/or B200GSR_BWD_PROJECT (accumulators -> parameter gradients);
- *   [g_begin, g_end) : the Gaussians the PROJECT stage covers (g_begin a multiple of 128).  The
- *               host issues COMPOSITE once, then PROJECT chunk by chunk, all-reducing finished chunks
- *               on a communication stream while the next chunk computes (dreamscene_b200.parallel);
- *               every Gaussian must be covered exactly once per backward (read-and-clear);
  *   dsh_coefs : 0 = d_shs has the reference layout [P, M, 3]; otherwise d_shs is a COMPACT
  *               [P, dsh_coefs, 3] array holding only the coefficients an active degree can touch
  *               ((sh_degree+1)^2 <= dsh_coefs <= M): the multi-GPU gradient payload at low degrees;
@@ -173,8 +167,6 @@ int b200gsr_backward(const b200gsr_params* prm,
  *               view is the outer product basis(view direction) x that vector, so ranks exchange 3 floats per
  *               Gaussian and view instead of 3*M and rebuild the sum with b200gsr_sh_grad_expand.
  */
-#define B200GSR_BWD_COMPOSITE 1u
-#define B200GSR_BWD_PROJECT 2u
 int b200gsr_backward_ex(const b200gsr_params* prm,
                         const float* means3D, const float* shs, const float* colors_precomp,
                         const float* opacities, const float* scales, const float* rotations,
@@ -185,8 +177,7 @@ int b200gsr_backward_ex(const b200gsr_params* prm,
                         uint64_t max_pairs,
                         float* d_means3D, float* d_means2D, float* d_shs, float* d_colors,
                         float* d_opacities, float* d_scales, float* d_rotations, float* d_cov3D,
-                        uint32_t stages, int32_t g_begin, int32_t g_end, int32_t dsh_coefs,
-                        void* stream);
+                        int32_t dsh_coefs, void* stream);
 
 /*
  * Sum of the SH gradients of `num_views` views from their factored form (additive; multi-GPU view sharding):

@@ -15,7 +15,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(b200gsr_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_of_abi_v4():
     from dreamscene_b200 import _build, _lib
     _build.build()
     lib = _lib.load()
@@ -23,7 +23,7 @@ def test_library_exports_every_declared_symbol():
     assert set(_lib.EXPORTS) == set(syms)
     for s in syms:
         assert hasattr(lib, s), s
-    assert lib.b200gsr_version() == 3
+    assert lib.b200gsr_version() == 4
 
 
 def test_layout_queries_are_monotone_and_aligned():

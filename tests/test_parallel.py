@@ -48,13 +48,11 @@ def _gloo_worker(rank, world, port, q):
     untouched = grads[rank].clone()
     parallel.maybe_all_reduce(untouched)
     ok = ok and torch.equal(untouched, grads[rank]) and uneven_refused
-    # the factored SH exchange is the default of the in-backward reduction (one chunk, <= 64 ranks)
+    # the factored SH exchange is the default of the in-backward reduction (<= 64 ranks)
     parallel.enable_view_sharding()
     ok = ok and parallel.factored_sh_exchange()
     parallel.enable_view_sharding(sh_exchange="dense")
     ok = ok and parallel.reduction_active() and not parallel.factored_sh_exchange()
-    parallel.enable_view_sharding(chunks=3)
-    ok = ok and not parallel.factored_sh_exchange()
     try:
         parallel.enable_view_sharding(sh_exchange="sparse")
         ok = False
@@ -84,7 +82,7 @@ def _gloo_worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_view_sharding_host_logic_gloo_world2():
+def test_view_sharding_host_logic_without_chunking_gloo_world2():
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
@@ -111,15 +109,14 @@ def _nccl_worker(rank, world, port, q):
     results = {}
 
     def view_grads(view, deg, mode, noise_seed=None):
-        """mode: 'backward' (in-backward chunked reduction), 'off' (no reduction), 'deferred' (leaf grads reduced
-        afterwards).  noise_seed: scene_render-style scale/SH augmentation between leaves and rasterizer."""
+        """mode: 'factored' / 'dense' (in-backward reduction with that SH exchange), 'off' (no reduction),
+        'deferred' (leaf grads reduced afterwards).  noise_seed: scene_render-style scale/SH augmentation
+        between leaves and rasterizer."""
         cam = U.cameras.orbit_camera(phi_deg=45.0 * view, height=256, width=256)
         S = U.cuda_settings(cam, deg, device=dev)
         t = {k: v.to(dev).requires_grad_(True) for k, v in sc.items()}
         m2d = torch.zeros(P, 3, device=dev, requires_grad=True)
-        if mode == "backward":
-            parallel.enable_view_sharding(chunks=3)                  # chunk-pipelined dense all-reduce
-        elif mode == "factored":
+        if mode == "factored":
             parallel.enable_view_sharding()                          # default: factored SH exchange (all-gather + expand)
         elif mode == "dense":
             parallel.enable_view_sharding(sh_exchange="dense")       # one all-reduce of the flat buffer incl. SH rows
@@ -144,7 +141,7 @@ def _nccl_worker(rank, world, port, q):
     for deg in (3, 1, 0):       # degree < 3: only the active SH columns travel (compact payload)
         seq = sum(view_grads(v, deg, "off")[0] for v in range(world))       # sequential loop on one GPU
         _, m2d_seq = view_grads(rank, deg, "off")
-        for mode in ("backward", "factored", "dense"):
+        for mode in ("factored", "dense"):
             reduced, m2d_own = view_grads(rank, deg, mode)
             err = float((reduced - seq).norm() / seq.norm())
             # per-view means2D grads are NOT reduced (equal up to the fp32 atomic summation order)
@@ -179,17 +176,6 @@ def test_view_sharded_backward_matches_sequential_sum_nccl():
     for p in procs:
         p.join(timeout=60)
     assert all(r[1] for r in res), res
-
-
-def test_chunk_bounds_cover_the_range_with_aligned_starts():
-    from dreamscene_b200 import parallel
-    for P in (1, 127, 128, 129, 1000, 1_000_000, 2_627_680):
-        for chunks in (1, 3, 8):
-            b = parallel.chunk_bounds(P, chunks)
-            assert b[0][0] == 0 and b[-1][1] == P and len(b) <= chunks
-            assert all(g0 % 128 == 0 and g0 < g1 for g0, g1 in b)
-            assert all(b[i][1] == b[i + 1][0] for i in range(len(b) - 1))
-    assert parallel.chunk_bounds(0) == []
 
 
 def test_sh_gradient_of_one_view_is_rank_one_per_gaussian_cpu_oracle():
